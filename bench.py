@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- stream-updates/s of the Precise streaming-inference hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--streams-per-gpu S] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--streams-per-gpu S] [--impl b200|reference] [--dump-outputs DIR]
 
 One "step" = one tick: every stream on the GPU receives one 1024-sample (2048-byte) chunk and is
 fully classified: PCM -> MFCC frames -> 29-step GRU scan -> sigmoid -> threshold decode -> trigger
@@ -36,6 +36,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True    # the benchmark leaves the tree as it found it (which may be read-only): no __pycache__ from its imports
 
 CHUNK = 1024
 PRIME = 24                # ticks that fill a 29-frame window: (24 * 1024 - 1600) // 800 + 1 = 29 frames
@@ -368,6 +369,20 @@ class ClockSampler:
 
 
 # ------------------------------------------------------------------------------------ GPU arm
+DUMP_MAX_STREAMS = 1 << 21      # 24 B of .npy data per stream: a dump stays under 48 MB at any --streams-per-gpu
+
+
+def last_tick_outputs(out, count):
+    """Host copies of what one StreamBatch.update tick returns to its caller (raw network output, decoded confidence and trigger
+    flag per stream) and of the detection count it accumulates.  Above DUMP_MAX_STREAMS streams a fixed, seeded sample of the
+    streams is kept; ``stream`` holds the stream index of every row."""
+    n = out['conf'].shape[0]
+    idx = np.arange(n) if n <= DUMP_MAX_STREAMS else np.sort(np.random.RandomState(0).choice(n, DUMP_MAX_STREAMS, replace=False))
+    return {'raw': out['raw'].cpu().numpy()[idx].astype(np.float32), 'conf': out['conf'].cpu().numpy()[idx].astype(np.float64),
+            'fired': out['fired'].cpu().numpy()[idx].astype(np.float32), 'stream': idx.astype(np.float64),
+            'detections': count.cpu().numpy().astype(np.float64)}
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -425,9 +440,10 @@ def run_b200(args):
     def step(t):
         if flush is not None:
             flush.add_(1)                      # rewrite 256 MB: evicts L2 between iterations
-        sb.update(dev_ticks[t % NT])
+        out = sb.update(dev_ticks[t % NT])
         if world > 1:
             counter.all_reduce_overlapped()    # snapshot on this stream, NCCL on a side stream under the next tick's K1
+        return out
 
     # ---- value: inputs resident in HBM
     # Priming (untimed, before the warm-up): PRIME ticks fill every stream's 29-frame window, so that each timed update
@@ -452,10 +468,12 @@ def run_b200(args):
         barrier()
     e0.record()
     for t in range(K):
-        step(W + t)
+        out = step(W + t)
     counter.wait()                              # the last tick's all-reduce is inside the timed region
     e1.record()
     barrier()
+    # the last timed tick's results, copied before the e2e loop below advances the same streams
+    dump = last_tick_outputs(out, counter.total if world > 1 else sb.count) if args.dump_outputs and rank == 0 else None
     ms = e0.elapsed_time(e1) - flush_ms
     kms, klaunch = core.profile_read()
     core.profile(False)
@@ -651,6 +669,8 @@ def run_b200(args):
     }
     if big:
         big.pop('k2_fp32_frac', None)
+    for name, a in (dump or {}).items():
+        np.save(os.path.join(args.dump_outputs, name + '.npy'), a)
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -671,7 +691,15 @@ def main():
     ap.add_argument('--no-numa-bind', action='store_true', help='do not pin the process to the CPUs of its GPU\'s NUMA node')
     ap.add_argument('--gru-mode', type=int, default=0, help='debug: 0 auto, 1 CUDA-core, 2 mma.sync, 3 tcgen05, 7 mma.sync with 32-stream tiles')
     ap.add_argument('--k1-mode', type=int, default=0, help='debug (A/B runs only): 0 default MFCC kernel choice, 2 FFT kernel, 3 FFT kernel with 64-bit set-up, 4 tcgen05 stage 2 only, 5 both DFT stages on tcgen05')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps write what the last one returned (rank 0\'s streams) as DIR/<name>.npy: '
+                    'raw, conf, fired, stream (the stream index of each row; a seeded sample above %d streams) and detections' % DUMP_MAX_STREAMS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs:
+        if args.impl != 'b200':
+            ap.error('--dump-outputs writes the outputs of the b200 arm')
+        os.makedirs(args.dump_outputs, exist_ok=True)
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == 'reference':
